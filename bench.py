@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — mel-frames/sec of the F5TTS.sample() hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one F5TTS.sample() ODE solve of one batch of synthetic utterances per GPU
@@ -23,6 +23,9 @@ utterance = 937 mel frames (328 ref + 609 gen), 152 text tokens, Euler, steps=32
                installable here) timed on this box's host cores on a bounded sample of the SAME
                workload
   --impl reference : times only that CPU restatement (rank 0), same metric/config.
+  --steps K  : timed steps of the headline, of e2e and of the FP8 mode (configs 3 and 5 time 2 and 3 steps)
+  --dump-outputs DIR : what the last timed step of each of them returned, as DIR/<name>.npy (see dump_outputs);
+               inputs and weights are seeded, so two builds run with the same arguments compare output for output
 """
 from __future__ import annotations
 
@@ -318,6 +321,10 @@ def measure(f5, lib, wl: Workload, rank: int, world: int, dev, steps: int, warmu
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    # what sample() returns for the last timed step: the final ODE state and the mel with the reference frames put back
+    state = plan.y[:, :N].clone()
+    mel = state.clone()
+    mel[:, :NR] = cond_d
     clk = clocks.stop() if clocks is not None else None
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -364,6 +371,7 @@ def measure(f5, lib, wl: Workload, rank: int, world: int, dev, steps: int, warmu
     if clk is not None:
         res["clocks"] = clk
     res["_inputs"] = (cond, text, y0, kw)
+    res["_outputs"] = {"mel": mel, "trajectory": state[None]}
     return res
 
 
@@ -420,9 +428,10 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
     clocks = ClockSampler(local_rank)
     m = measure(f5, lib, main_wl, rank, world, dev, args.steps, args.warmup, clocks)
     cond, text, y0, kw = m.pop("_inputs")
+    outputs = m.pop("_outputs")
 
     # ---- end to end through the public API with HOST buffers (same batch as the headline) ----
-    e2e_steps = max(2, min(args.steps, 10))
+    e2e_steps = args.steps
     y0_h = y0.contiguous().pin_memory()
     if B == 1:
         audio_h = synth_audio(REF_SAMPLES if NR == REF_SAMPLES // HOP else NR * HOP, seed=7 + rank).pin_memory()
@@ -447,6 +456,7 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
         w = e2e_once()
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
+    outputs["e2e_wave"] = w
     te = torch.tensor([e2e_s], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(te, op=dist.ReduceOp.MAX)
@@ -462,6 +472,7 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
             f5._plans.clear(); model._sessions.clear(); torch.cuda.empty_cache()
             r = measure(f5, lib, wl, rank, world, dev, st, 1)
             r.pop("_inputs")
+            outputs[wl.name + "_mel"] = r.pop("_outputs")["mel"]
             subs[wl.name] = r
         # config 4 of BASELINE.json (512 utterances over 8 GPUs = 64 per GPU, weights broadcast once, no per-step
         # collective) is cfg3_b64_midpoint at --gpus 8: its `value` is the whole-job aggregate over all ranks
@@ -480,8 +491,9 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
             if world > 1:
                 m8.packed.broadcast(src=0)
             r = measure(F5TTS(m8), lib, Workload("b1_fp8", B, N, NR, args.method, args.ode_steps, args.cfg), rank, world, dev,
-                        max(3, min(args.steps, 10)), 3)
+                        args.steps, 3)
             r.pop("_inputs")
+            outputs["b1_fp8_mel"] = r.pop("_outputs")["mel"]
             r["dtype"] = "fp8 (e4m3 operands of QKV / out / FF1 / FF2, fp32 accumulate) + bf16 elsewhere"
             r["note"] = "lossy mode: oracle-emulated drift 2.9e-2 per forward vs 3.9e-3 for bf16 (DESIGN.md section 8)"
             subs["b1_fp8"] = r
@@ -512,7 +524,29 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
             "roofline": m["roofline"], "cpu_baseline": cpu, "rtf": m["rtf"],
             "generated_frames_per_s": m["generated_frames_per_s"], "fused_adaln": not args.no_fused_adaln,
             "configs": subs}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes rank 0's outputs of the last timed step as <out_dir>/<name>.npy in float32, DUMP_BYTES at most in all:
+    the smaller arrays are written whole, and one whose share of what is left is too small is replaced by a fixed,
+    seeded sample of its elements (flattened, in index order), so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(items):
+        a = t.detach().float().cpu().numpy()
+        keep = (left // (len(items) - i) - 128) // a.itemsize           # 128: the .npy header
+        if a.size > keep:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        left -= os.path.getsize(path)
 
 
 def main():
@@ -533,7 +567,12 @@ def main():
     ap.add_argument("--fp8", action="store_true", help="FP8 mode (e4m3 QKV / FF1 GEMMs): the lossy analogue of the reference's --q; "
                                                         "NOT the headline (dtype is reported as fp8+bf16)")
     ap.add_argument("--profile-run", action="store_true", help="one eager step and exit (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (mel, trajectory, e2e_wave, <config>_mel) "
+                         "as DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.profile_run):
+        ap.error("--dump-outputs applies to the timed CUDA arm")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

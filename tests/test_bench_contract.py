@@ -38,6 +38,27 @@ def test_reference_arm_prints_one_contract_line():
     assert abs(d["value"] - 937 / (d["ms_per_step"] / 1e3 * 15.5)) / d["value"] < 1e-6
 
 
+def test_dump_outputs_is_reproducible_and_stays_within_its_budget(tmp_path, monkeypatch):
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200_000)
+    small = torch.arange(1000, dtype=torch.float64).reshape(10, 100)
+    big = torch.randn(3, 50_000, generator=torch.Generator().manual_seed(0))
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"big": big, "small": small})
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 200_000
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, small.float().numpy())          # written whole
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and 0 < a.size < big.numel() and np.array_equal(a, b)  # the same sample every run
+    assert np.isin(a, big.numpy().ravel()).all()
+    r = _run("--impl", "reference", "--dump-outputs", str(tmp_path / "c"))
+    assert r.returncode != 0 and not (tmp_path / "c").exists()
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
 def test_cuda_arm_fails_loudly_without_a_gpu():
     r = _run("--steps", "1", "--warmup", "0", timeout=300)

@@ -302,7 +302,7 @@ def test_full_size_golden_fixtures_present_and_inputs_reproducible(golden_dir):
     G = importlib.util.module_from_spec(spec); spec.loader.exec_module(G)
     for name, fn, keys in (("full_cfg2_sample", G.inputs_cfg2, {"out": (1, 937, 100), "traj_mid": (1, 937, 100)}),
                            ("full_cfg3_sample", G.inputs_cfg3, {"out_0": (937, 100), "out_37": (937, 100)}),
-                           ("full_cfg5_long", G.inputs_cfg5, {"out_sub3": (1875, 100), "fwd_sub3": (1875, 100)})):
+                           ("full_cfg5_long", G.inputs_cfg5, {"out_sub6": (938, 100), "fwd_sub6": (938, 100)})):
         z = np.load(os.path.join(golden_dir, name + ".npz"))
         for k, shp in keys.items():
             assert z[k].shape == shp and np.isfinite(z[k]).all(), (name, k, z[k].shape)
